@@ -14,7 +14,10 @@ optimised pose back every frame. N > 1 = N independent streams, one per GPU (BAS
 "replicas only", no data-path collective), value = total frames / max-over-ranks time.
 
 `--impl reference` times the reference's own CPU arithmetic (the oracle port, see oracle/) with all host
-threads on a bounded sample of the same workload.
+threads on `--steps` frames of the same workload (about 10 s per frame).
+
+`--dump-outputs DIR` writes what the timed GPU path returned for its last step (bench.dump_outputs); the inputs are
+seeded, so two builds run with the same arguments can be compared array for array.
 """
 from __future__ import annotations
 
@@ -184,7 +187,25 @@ def time_corr_kernel(device: str, iters: int = 10) -> dict:
     return {"seconds": sum(times) / len(times), "bytes": algo_bytes, "mode": ops.CORR_MODE_NAMES[mode]}
 
 
-def run_gpu(cfg: dict, steps: int, warmup: int, n_gpus: int) -> dict:
+def dump_outputs(odo, out_dir: str) -> None:
+    """What the fused driver hands its caller for the last timed frame — the optimised pose, the frame's packed observations
+    and mapping points — plus the whole trajectory, as <name>.npy (float32 / float64, counts as 1-element arrays); well under
+    1 MB for every config. An array with no rows is not written: it holds nothing to compare (on the synthetic sequence no
+    pixel passes the mapping selector's depth gates, so the mapping points are empty)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"pose": odo.latest_pose(), "trajectory": odo.finish()}
+    for k, v in odo.observations().items():
+        arrays[k] = torch.as_tensor(v).reshape(-1) if not torch.is_tensor(v) else v
+    for k, v in arrays.items():
+        v = v.detach().cpu()
+        if v.numel() == 0:
+            continue
+        v = v.double() if v.dtype in (torch.float64, torch.int64, torch.int32) else v.float()
+        np.save(os.path.join(out_dir, f"{k}.npy"), v.numpy())
+
+
+def run_gpu(cfg: dict, steps: int, warmup: int, n_gpus: int, dump_dir: str | None = None) -> dict:
     rank, world, local = _dist()
     assert torch.cuda.is_available(), "bench.py (GPU arm) needs CUDA; use --impl reference for the CPU arm"
     torch.cuda.set_device(local)
@@ -250,7 +271,10 @@ def run_gpu(cfg: dict, steps: int, warmup: int, n_gpus: int) -> dict:
         return ms, ops.LAUNCHES[0], odo
 
     with ClockSampler(local) as clk:
-        ms_dev, launches, _ = timed(frames_dev, read_pose=False)
+        ms_dev, launches, odo_dev = timed(frames_dev, read_pose=False)
+        if dump_dir and rank == 0:
+            dump_outputs(odo_dev, dump_dir)
+        del odo_dev
         ms_e2e, _, _ = timed(frames_host, read_pose=True)
         ms_api, _, _ = timed(frames_host, read_pose=True, fused=False)
     corr = time_corr_kernel(device)
@@ -309,7 +333,7 @@ def run_gpu(cfg: dict, steps: int, warmup: int, n_gpus: int) -> dict:
     return out if rank == 0 else {}
 
 
-def run_sharded(steps: int, warmup: int) -> dict:
+def run_sharded(steps: int, warmup: int, dump_dir: str | None = None) -> dict:
     """BASELINE configs[3]: ONE 1280x720 stream, 4096 keypoints, on N GPUs. Rank 0 owns the frontend, the selection and the
     device-side observation building; per frame it broadcasts the five LM input arrays (NCCL, 80 B per keypoint slot) and
     every rank solves its shard of residual blocks with the all-reduce of the 55-double accumulator fused into the persistent
@@ -388,6 +412,8 @@ def run_sharded(steps: int, warmup: int) -> dict:
         gathered = [torch.zeros_like(mine) for _ in range(world)]
         dist.all_gather(gathered, mine)
         poses_equal = all(torch.equal(g, gathered[0]) for g in gathered)
+    if dump_dir and rank == 0:
+        dump_outputs(odo, dump_dir)
     out = {}
     if rank == 0:
         o = odo.observations()
@@ -419,11 +445,17 @@ def main() -> None:
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--config", default="performant", choices=list(CONFIGS) + ["sharded"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path returned for its last step as DIR/<name>.npy (GPU arm)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs applies to the GPU arm (--impl b200)")
     a.warmup = max(a.warmup, 3) if a.impl == "b200" else a.warmup
     rank, world, _ = _dist()
     if a.config == "sharded":
-        out = run_sharded(a.steps, a.warmup)
+        out = run_sharded(a.steps, a.warmup, a.dump_outputs)
         if rank == 0:
             print(json.dumps(out), flush=True)
         return
@@ -431,19 +463,19 @@ def main() -> None:
     if a.impl == "reference":
         if rank != 0:
             return                                   # rank 0 alone runs the CPU arm
-        steps = max(1, min(a.steps, 2))              # bounded sample: ~10 s per 640x480 frame on 8 cores
+        steps = a.steps                              # ~10 s per 640x480 frame on 8 cores
         warm = min(a.warmup, 1)
         r = run_cpu(cfg, frames_to_time=steps, warm=warm)
         line = {"impl": "reference", "metric": METRIC, "value": r["value"], "unit": "frames/s", "n_gpus": a.gpus,
                 "steps": steps, "warmup": warm, "ms_per_step": 1e3 / r["value"], "higher_is_better": True,
                 "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
                 "config": {"workload": workload_name(cfg),
-                           "arm": "CPU arithmetic of the reference (oracle port; the reference tree cannot travel to the GPU box), "
-                                  "bounded sample of the same workload"},
+                           "arm": "CPU arithmetic of the reference (oracle port), "
+                                  f"{steps} frame(s) of the same workload"},
                 "cpu_baseline": r, "e2e": {"value": r["value"], "unit": "frames/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
         print(json.dumps(line), flush=True)
         return
-    out = run_gpu(cfg, a.steps, a.warmup, a.gpus)
+    out = run_gpu(cfg, a.steps, a.warmup, a.gpus, a.dump_outputs)
     if rank == 0:
         print(json.dumps(out), flush=True)
 

@@ -1,7 +1,7 @@
-"""TEST INFRASTRUCTURE: import the read-only MAC-VO reference (`/root/reference`) in this container.
+"""TEST INFRASTRUCTURE: import the read-only MAC-VO reference tree (MACVO_REFERENCE_ROOT).
 
-Used only by `tests/golden/make_golden.py` (fixture generation) and by tests that are skipped when
-`/root/reference` is absent (it never exists on the GPU box). Nothing in the product imports this.
+Used only by the fixture generators `tests/golden/make_golden*.py`; the tests read the fixtures they
+write and never need the tree. Nothing in the product imports this.
 
 * `yacs` is absent -> tiny `CfgNode` stand-in (`refharness/yacs`).
 * `pypose` is absent -> functional restatement (`oracle/pypose_shim`).

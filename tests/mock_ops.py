@@ -1,8 +1,8 @@
 """TEST INFRASTRUCTURE: oracle-backed CPU stand-ins for the C-ABI calls in `macvo_b200.ops`.
 
 Purpose: run the HOST logic of the five B200 plugin classes (config handling, adapters, tensor shapes / dtypes / devices,
-`GraphInput -> PGOInput`, the in-place side effects MAC-VO relies on) under the REAL `Odometry/MACVO.py` in the build
-container, which has the reference tree but no GPU (tests/test_macvo_integration.py). Every kernel call is answered by
+`GraphInput -> PGOInput`, the in-place side effects MAC-VO relies on) without a GPU, against a recorded run of
+`Odometry/MACVO.py` (tests/test_macvo_integration.py). Every kernel call is answered by
 the CPU oracle that the GPU parity tests pin the kernels to. Never imported by the product.
 """
 from __future__ import annotations

@@ -48,7 +48,7 @@ def _worker(rank: int, world: int, port: int, out_q):
     dist.destroy_process_group()
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
 @pytest.mark.parametrize("world", [2, 4])
 def test_fused_sharded_pgo_matches_single_gpu_and_oracle(world):
     if torch.cuda.device_count() < world:

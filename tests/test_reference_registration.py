@@ -1,60 +1,39 @@
-"""Drop-in check against the REAL MAC-VO tree (build container only; skipped where /root/reference is absent):
-importing `macvo_b200.plugins` with MAC-VO importable registers the B200 classes in MAC-VO's own registries,
-`Module.I<X>.instantiate` finds them by name and `is_valid_config` accepts the INTEGRATION.md YAML args.
-Runs in a subprocess so that the reference import does not leak into the other tests."""
-import os
-import subprocess
-import sys
+"""Drop-in check against MAC-VO's own registry and config specs, recorded from the MAC-VO tree in
+tests/golden/macvo_registry.pt (tests/golden/make_golden_macvo.py): for each module of MACVO_Performant.yaml that a B200 class
+replaces, the interface MAC-VO files it under, the keys its `is_valid_config` demands and the YAML's args. Each B200 class
+must be found by name under the interface of that name, accept the same args (on a CUDA device) through the
+interface-level validator `MACVO.is_valid_config` calls (Odometry/MACVO.py:137-156), require every key the replaced class
+requires and reject an excess key like it."""
+from types import SimpleNamespace as NS
 
 import pytest
 
-from tests.golden import refharness
-
-REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
-CODE = r'''
-import sys
-sys.path.insert(0, %r)
-from tests.golden import refharness
-refharness.install()
-from types import SimpleNamespace as NS
-import Module
-import macvo_b200.plugins as P
-assert P._REF, "plugins did not detect the MAC-VO tree"
-from Module import IFrontend, IKeypointSelector, ICovariance2to3, IOptimizer
-assert IFrontend.get_class("B200_FlowFormerCovFrontend") is P.B200_FlowFormerCovFrontend
-assert IKeypointSelector.get_class("B200_CovAwareSelector_NoDepth") is P.B200_CovAwareSelector_NoDepth
-assert IKeypointSelector.get_class("B200_MappingPointSelector") is P.B200_MappingPointSelector
-assert ICovariance2to3.get_class("B200_MatchCovariance") is P.B200_MatchCovariance
-assert IOptimizer.get_class("B200_TwoFrame_PGO") is P.B200_TwoFrame_PGO
-from Module.Optimization.TwoFramePGO.Optimizer import TwoFrame_PGO
-assert issubclass(P.B200_TwoFrame_PGO, TwoFrame_PGO)
-# the interface-level validators MACVO.is_valid_config calls (Odometry/MACVO.py:137-156)
-IFrontend.is_valid_config(NS(type="B200_FlowFormerCovFrontend", args=NS(device="cuda", weight="./Model/MACVO_FrontendCov.pth",
-    enc_dtype="fp32", dec_dtype="fp32", decoder_depth=12, enforce_positive_disparity=False, cuda_graph=True)))
-IKeypointSelector.is_valid_config(NS(type="B200_CovAwareSelector_NoDepth", args=NS(device="cuda", kernel_size=7, mask_width=32, max_match_cov=100.0)))
-IKeypointSelector.is_valid_config(NS(type="B200_MappingPointSelector", args=NS(max_depth=5.0, max_depth_cov=0.005, mask_width=32)))
-ICovariance2to3.is_valid_config(NS(type="B200_MatchCovariance", args=NS(device="cuda", kernel_size=31, match_cov_default=0.25, min_depth_cov=0.05, min_flow_cov=0.25)))
-IOptimizer.is_valid_config(NS(type="B200_TwoFrame_PGO", args=NS(device="cuda", vectorize=True, parallel=False, graph_type="disp", autodiff=False)))
-try:
-    IKeypointSelector.is_valid_config(NS(type="B200_CovAwareSelector_NoDepth", args=NS(device="cuda", kernel_size=7, mask_width=32, max_match_cov=100.0, extra=1)))
-    raise SystemExit("excess key accepted")
-except KeyError:
-    pass
-try:
-    P.B200_MatchCovariance(NS(device="cpu", kernel_size=31, match_cov_default=0.25, min_depth_cov=0.05, min_flow_cov=0.25))
-    raise SystemExit("cpu device accepted")
-except ValueError:
-    pass
-print("REGISTERED-OK")
-''' % REPO
+B200 = {"frontend": "B200_FlowFormerCovFrontend", "keypoint": "B200_CovAwareSelector_NoDepth",
+        "mappoint": "B200_MappingPointSelector", "cov": "B200_MatchCovariance", "optimizer": "B200_TwoFrame_PGO"}
 
 
-@pytest.mark.skipif(not refharness.available(), reason="MAC-VO reference tree not present")
-def test_plugins_register_into_macvo_registry():
-    r = subprocess.run([sys.executable, "-c", CODE], capture_output=True, text=True, timeout=600,
-                       env=dict(os.environ, TORCHDYNAMO_DISABLE="1"))
-    assert "REGISTERED-OK" in r.stdout, r.stdout[-2000:] + r.stderr[-3000:]
+def test_plugins_register_into_macvo_registry(golden):
+    from macvo_b200 import plugins as P
+    ref = golden("macvo_registry.pt")
+    assert set(ref) == set(B200)
+    for role, name in B200.items():
+        r, cls = ref[role], getattr(P, name)
+        iface = next(c for c in cls.__mro__ if c.__name__ == r["interface"])
+        assert iface.get_class(name) is cls, (role, r["interface"])
+        args = dict(r["args"])
+        if "device" in args:
+            args["device"] = "cuda"
+        if role == "optimizer":
+            args["parallel"] = False            # the B200 optimiser's asynchrony is its CUDA stream, not a spawned process
+        iface.is_valid_config(NS(type=name, args=NS(**args)))
+        for key in r["spec_keys"]:
+            with pytest.raises(KeyError):
+                cls.is_valid_config(NS(**{k: v for k, v in args.items() if k != key}))
+        assert r["excess_rejected"]
+        with pytest.raises(KeyError):
+            iface.is_valid_config(NS(type=name, args=NS(**args, extra=1)))
+    with pytest.raises(ValueError):
+        P.B200_MatchCovariance(NS(device="cpu", kernel_size=31, match_cov_default=0.25, min_depth_cov=0.05, min_flow_cov=0.25))
 
 
 def test_local_interfaces_registry_and_config_spec():
